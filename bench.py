@@ -37,6 +37,10 @@ map (~190.8 GB of 191.5 GB), poisoned with 0xA5 before the first step.
             NUMA-local first touch, pinned threads.
 
 Other modes:  --sweep  region sweep 1 GB -> max (BASELINE configs[4]) on this rank's GPU.
+
+--dump-outputs DIR  after the timed steps, runs the step once more on a seeded dirty input and
+            writes what it computed to DIR as .npy (see dump_outputs), so that two builds can be
+            compared output for output.
 """
 from __future__ import annotations
 
@@ -240,6 +244,44 @@ def injected_count_check(L, N, dev, R, vv, sptr):
     return {"injected": 7, "counted": found, "after_scrub": nz.value, "offsets_include": ["first byte", "last byte", "unaligned"]}
 
 
+DUMP_WINDOWS, DUMP_WINDOW_BYTES, DUMP_SEED = 64, 16 << 10, 42
+
+
+def dump_outputs(L, dev, R, vv, sptr, step, out_dir, rank=None):
+    """Runs the timed step once more on a seeded input and writes what it computed to out_dir.
+
+    A correct step always ends with a zeroed arena and a count of 0, so the timed steps' own results
+    cannot tell a verify kernel that counts from one that always says 0.  The step is therefore given
+    dirt it must see: the arena is filled with the seeded xorshift pattern (ccm_arena_fill_random,
+    seed 42; the same arguments give the same input on every run), counted with the step's verify
+    kernel, and then scrubbed and verified by the timed call itself.  Files (.npy):
+      input_nonzero_bytes  non-zero bytes the verify kernel counts in the seeded input (float64)
+      nonzero_bytes        the count the step hands its caller (ccm_arena_fetch_count; float64)
+      arena_sample         the scrubbed arena, float32, one row per window: the first and last
+                           16 KiB and 64 windows of 16 KiB at offsets drawn with seed 0
+    Under torchrun every rank writes its own files, suffixed _rank<r>."""
+    import numpy as np
+    nz = C.c_uint64()
+    check(L.ccm_arena_fill_random(dev, DUMP_SEED, sptr), "fill seeded input")
+    check(L.ccm_arena_verify(dev, vv, None, sptr, C.byref(nz), None), "verify seeded input")
+    dirty = nz.value
+    step()
+    check(L.ccm_arena_fetch_count(dev, sptr, C.byref(nz)), "fetch_count")
+    if dirty == 0 or nz.value != 0:
+        raise RuntimeError(f"seeded input counted {dirty} non-zero bytes, {nz.value} after the step")
+    w = min(DUMP_WINDOW_BYTES, R)
+    rng = np.random.default_rng(0)
+    offsets = [0, R - w] + sorted(int(x) for x in rng.integers(0, R - w + 1, size=DUMP_WINDOWS))
+    sample = np.empty((len(offsets), w), dtype=np.uint8)
+    for row, off in zip(sample, offsets):
+        check(L.ccm_arena_read(dev, off, row.ctypes.data, w), "arena_read")
+    suffix = "" if rank is None else f"_rank{rank}"
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / f"input_nonzero_bytes{suffix}.npy", np.array([dirty], dtype=np.float64))
+    np.save(out_dir / f"nonzero_bytes{suffix}.npy", np.array([nz.value], dtype=np.float64))
+    np.save(out_dir / f"arena_sample{suffix}.npy", sample.astype(np.float32))
+
+
 def run_ours(args):
     import torch
 
@@ -341,6 +383,8 @@ def run_ours(args):
     check(L.ccm_arena_step_times(dev, 64, s_ms, v_ms, C.byref(nsteps)), "step_times")
     scrub_ms = statistics.mean(s_ms[:nsteps.value]) if nsteps.value else float("nan")
     verify_ms = statistics.mean(v_ms[:nsteps.value]) if nsteps.value else float("nan")
+    if args.dump_outputs:                                       # after the step times: its step is not timed
+        dump_outputs(L, dev, R, vv, sptr, step, Path(args.dump_outputs), rank if world > 1 else None)
 
     # ---- same-run peaks: the library write bar over the same arena ... ------------------
     peaks = {}
@@ -897,6 +941,7 @@ def main():
     ap.add_argument("--no-baselines", action="store_true")
     ap.add_argument("--no-node-leg", action="store_true")
     ap.add_argument("--no-host-roundtrip", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/*.npy")
     ap.add_argument("--sweep", action="store_true", help="region sweep 1 GB -> max instead of the bench line")
     ap.add_argument("--cpu-probe", action="store_true", help="only the CPU arm, with its tuning table")
     ap.add_argument("--node-leg", action="store_true", help=argparse.SUPPRESS)

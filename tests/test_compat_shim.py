@@ -1,24 +1,23 @@
 """The gpu-admin-tools-shaped shim: the UNMODIFIED reference main.py runs on libccm.so.
 
-The reference itself is only present in the development container; that part of the test
-skips on the GPU box.  The CLI twin (reference scripts/cc-manager.sh:127,389) is always tested."""
+What the reference calls through the shim, and what each call returned, is recorded in
+tests/golden/reference_shim_calls.json (oracle/gen_shim_calls.py); the test replays it against the
+shim.  The CLI twin (reference scripts/cc-manager.sh:127,389) is tested as well."""
 from __future__ import annotations
 
-import importlib.util
 import json
-import os
 import sys
 from pathlib import Path
 
 import pytest
 
 import scenarios as SC
-from helpers import build_native_world, build_cluster, k8s_trace, registers, sim_trace, sim_trace_clear
+from helpers import build_native_world, registers, sim_trace, sim_trace_clear
 
 ROOT = Path(__file__).resolve().parents[1]
 COMPAT = ROOT / "k8s_cc_manager_b200" / "compat" / "gpu-admin-tools"
-REFERENCE = Path(os.environ.get("CCM_REFERENCE_DIR", "/root/reference"))
 GOLDEN = {s["name"]: s for s in json.loads((ROOT / "tests/golden/transitions.json").read_text())["scenarios"]}
+SHIM_CALLS = {s["name"]: s for s in json.loads((ROOT / "tests/golden/reference_shim_calls.json").read_text())["scenarios"]}
 
 
 def test_cli_twin_prints_what_the_shell_engine_parses(capsys):
@@ -38,43 +37,47 @@ def test_cli_twin_prints_what_the_shell_engine_parses(capsys):
         sys.modules.pop("nvidia_gpu_tools", None)
 
 
-@pytest.mark.skipif(not (REFERENCE / "main.py").exists(), reason="reference checkout only exists in the dev container")
 @pytest.mark.parametrize("name", ["off_to_on_evict_pods_gone", "roundtrip_on_devtools_off", "cc_on_with_ppcie_active",
                                   "ppcie_from_off", "fault_set_gpuerror_gpu3", "fault_stuck_mode_gpu5",
                                   "get_only_8gpu_on"])
 def test_unmodified_reference_runs_on_libccm(name, monkeypatch):
-    """Drop-in check: reference main.py + reference gpu_operator_eviction.py, device layer =
-    compat shim -> ctypes -> libccm.so (sim registers).  Same traces as with the fake
-    gpu-admin-tools the goldens were recorded with."""
+    """Drop-in check: the reference main.py's calls into the shim (device enumeration, attribute
+    reads, register ops), replayed in order against compat shim -> ctypes -> libccm.so (sim
+    registers), must return or raise what they did for the reference, and leave the same register
+    trace and end registers as the fake gpu-admin-tools the goldens were recorded with."""
     sc = next(s for s in SC.transition_scenarios() if s["name"] == name)
-    for mod in ("nvidia_gpu_tools", "pci", "pci.devices", "gpu", "gpu_operator_eviction"):
+    shim_modules = ("nvidia_gpu_tools", "pci", "pci.devices", "gpu")
+    for mod in shim_modules:
         sys.modules.pop(mod, None)
-    monkeypatch.syspath_prepend(str(REFERENCE))
     monkeypatch.syspath_prepend(str(COMPAT))
-    spec = importlib.util.spec_from_file_location("reference_main_on_libccm", REFERENCE / "main.py")
-    ref = importlib.util.module_from_spec(spec)
-    saved = list(sys.path)
-    spec.loader.exec_module(ref)
-    sys.path[:] = saved
-    import gpu_operator_eviction as ref_evict
-    assert Path(ref_evict.__file__).parent == REFERENCE
     try:
+        from gpu import GpuError
+        from nvidia_gpu_tools import Gpu  # noqa: F401 - imported by the reference (main.py:38)
+        from pci.devices import find_gpus
         build_native_world(sc)
-        c = build_cluster(sc)
-        ref_evict.time = c.clock
-        monkeypatch.setenv("EVICT_OPERATOR_COMPONENTS", "true" if sc["evict"] else "false")
-        monkeypatch.setenv("OPERATOR_NAMESPACE", SC.NAMESPACE)
-        mgr = ref.CCManager(node_name=SC.NODE, default_mode="on", host_cc=sc["host_cc"])
-        for mode, want in zip(sc["modes"], GOLDEN[name]["steps"]):
-            n_k8s = len(c.calls)
+        steps = SHIM_CALLS[name]["steps"]
+        assert [s["mode"] for s in steps] == sc["modes"]
+        for step, want in zip(steps, GOLDEN[name]["steps"]):
             sim_trace_clear()
-            assert mgr.set_cc_mode(mode) == want["result"]
+            devices, finds = {}, 0
+            for entry in step["calls"]:
+                if entry[0] == "find_gpus":
+                    devs, n = find_gpus()
+                    assert [len(devs), n] == entry[1:]
+                    devices.update({f"{finds}:{i}": d for i, d in enumerate(devs)})
+                    finds += 1
+                elif entry[1].endswith("()"):
+                    handle, method, args, outcome = entry
+                    try:
+                        got = {"return": getattr(devices[handle], method[:-2])(*args)}
+                    except GpuError as exc:
+                        got = {"raise": type(exc).__name__}
+                    assert got == outcome, (step["mode"], entry)
+                else:
+                    handle, attr, value = entry
+                    assert getattr(devices[handle], attr) == value, (step["mode"], entry)
             assert sim_trace() == want["device_trace"]
-            assert k8s_trace(c)[n_k8s:] == want["k8s"]
-            assert c.labels(SC.NODE) == want["labels"]
             assert registers() == want["registers"]
     finally:
-        for mod in ("nvidia_gpu_tools", "pci", "pci.devices", "gpu", "gpu_operator_eviction"):
+        for mod in shim_modules:
             sys.modules.pop(mod, None)
-        import time as real_time
-        ref_evict.time = real_time

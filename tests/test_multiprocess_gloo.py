@@ -129,3 +129,68 @@ def test_bench_b0_get_only_runs_on_the_sim_backend(native, cluster):
     assert out["gpus"] == 4 and 1.0 < out["product_us_median"] < 5000.0
     ref = out["reference_main_py_committed"]
     assert ref and ref["reference_fake_devices"] > 0 and ref["product_serial"] > 0
+
+
+def test_bench_dump_outputs_runs_the_step_on_a_seeded_input(tmp_path):
+    """--dump-outputs: seeded dirt counted by the step's verify kernel, the step's own count, and the same
+    seeded windows of the scrubbed arena on every run, well under 64 MB; a verify that sees no dirt fails."""
+    import ctypes as C
+
+    import numpy as np
+    import pytest
+    sys.path.insert(0, str(ROOT))
+    import bench
+    R = (3 << 30) + 5
+
+    class FakeArena:
+        """Arena of R bytes: the seeded fill makes it (offset % 251), the step zeroes it."""
+
+        def __init__(self, verify_sees_dirt=True):
+            self.calls, self.dirty, self.sees = [], False, verify_sees_dirt
+
+        def ccm_arena_fill_random(self, dev, seed, stream):
+            self.calls.append(("fill", seed))
+            self.dirty = True
+            return 0
+
+        def ccm_arena_verify(self, dev, variant, cfg, stream, nz, ms):
+            self.calls.append(("verify", variant))
+            nz._obj.value = R - R // 251 - 1 if self.dirty and self.sees else 0
+            return 0
+
+        def step(self):
+            self.calls.append(("step",))
+            self.dirty = False
+
+        def ccm_arena_fetch_count(self, dev, stream, nz):
+            nz._obj.value = 0
+            return 0
+
+        def ccm_arena_read(self, dev, off, dst, n):
+            self.calls.append(("read", off))
+            assert 0 <= off and off + n <= R
+            C.memmove(dst, bytes((off + i) % 251 if self.dirty else 0 for i in range(n)), n)
+            return 0
+
+    arenas = {d: FakeArena() for d in ("a", "b", "r")}
+    for d in ("a", "b"):
+        bench.dump_outputs(arenas[d], 0, R, 7, None, arenas[d].step, tmp_path / d)
+    bench.dump_outputs(arenas["r"], 1, R, 7, None, arenas["r"].step, tmp_path / "r", rank=1)
+    a = arenas["a"]
+    assert a.calls[:3] == [("fill", bench.DUMP_SEED), ("verify", 7), ("step",)]
+    load = lambda d, n: np.load(tmp_path / d / f"{n}.npy")  # noqa: E731
+    assert load("a", "input_nonzero_bytes").dtype == np.float64
+    assert load("a", "input_nonzero_bytes").tolist() == [R - R // 251 - 1] and load("a", "nonzero_bytes").tolist() == [0.0]
+    sample = load("a", "arena_sample")
+    assert sample.dtype == np.float32 and sample.shape == (bench.DUMP_WINDOWS + 2, bench.DUMP_WINDOW_BYTES)
+    assert not sample.any()                                          # read back after the step's scrub
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) < 64 << 20
+    for n in ("input_nonzero_bytes", "nonzero_bytes", "arena_sample"):
+        assert np.array_equal(load("a", n), load("b", n))
+    offs = [c[1] for c in a.calls if c[0] == "read"]
+    assert offs == [c[1] for c in arenas["b"].calls if c[0] == "read"]
+    assert offs[:2] == [0, R - bench.DUMP_WINDOW_BYTES] and len(set(offs)) == len(offs) == bench.DUMP_WINDOWS + 2
+    assert load("r", "input_nonzero_bytes_rank1").tolist() == [R - R // 251 - 1]
+    blind = FakeArena(verify_sees_dirt=False)
+    with pytest.raises(RuntimeError, match="seeded input counted 0"):
+        bench.dump_outputs(blind, 0, R, 7, None, blind.step, tmp_path / "blind")

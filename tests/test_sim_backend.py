@@ -122,6 +122,7 @@ def test_python_manager_wallclock_scales_with_max_not_sum(sim, monkeypatch):
 
 
 def test_sysfs_backend_enumerates_fake_tree(tmp_path, monkeypatch):
+    # PCI domain fffe: no host puts a real GPU there, so no CUDA device matches these addresses
     root = tmp_path / "devices"
 
     def dev(bdf, vendor, cls, device="0x2901"):
@@ -132,25 +133,26 @@ def test_sysfs_backend_enumerates_fake_tree(tmp_path, monkeypatch):
         (d / "device").write_text(device + "\n")
         (d / "reset").write_text("")
 
-    dev("0000:1b:00.0", "0x10de", "0x030200")
-    dev("0000:43:00.0", "0x10de", "0x030000")
-    dev("0000:05:00.0", "0x10de", "0x068000", "0x22a3")
-    dev("0000:00:1f.0", "0x8086", "0x060100")
-    dev("0000:aa:00.0", "0x10de", "0x0c0330")  # NVIDIA USB controller: not a GPU
+    dev("fffe:1b:00.0", "0x10de", "0x030200")
+    dev("fffe:43:00.0", "0x10de", "0x030000")
+    dev("fffe:05:00.0", "0x10de", "0x068000", "0x22a3")
+    dev("fffe:00:1f.0", "0x8086", "0x060100")
+    dev("fffe:aa:00.0", "0x10de", "0x0c0330")  # NVIDIA USB controller: not a GPU
     monkeypatch.setenv("CCM_SYSFS_ROOT", str(root))
     try:
         D.select_backend("sysfs")
         devs, n = D.find_gpus()
-        assert [(d.bdf, d.is_gpu()) for d in devs] == [("0000:05:00.0", False), ("0000:1b:00.0", True),
-                                                       ("0000:43:00.0", True)]
+        assert [(d.bdf, d.is_gpu()) for d in devs] == [("fffe:05:00.0", False), ("fffe:1b:00.0", True),
+                                                       ("fffe:43:00.0", True)]
         gpu = devs[1]
         with pytest.raises(D.GpuError) as e:   # register map is not part of this build
             gpu.set_cc_mode("on")
         assert e.value.status == N.ERR_UNSUPPORTED
         gpu.reset_with_os()
-        assert (root / "0000:1b:00.0" / "reset").read_text() == "1"
+        assert (root / "fffe:1b:00.0" / "reset").read_text() == "1"
         gpu.wait_for_boot(timeout_ms=200)
-        with pytest.raises(D.GpuError):        # no CUDA device behind it here
+        with pytest.raises(D.GpuError) as e:   # no CUDA device behind it here
             gpu.scrub_and_verify(1 << 20)
+        assert e.value.status == N.ERR_NO_CUDA
     finally:
         D.select_backend("sim")
